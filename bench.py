@@ -7,7 +7,8 @@ one stream per block), i.e. one full round trip of the rank's data through the r
   e2e        MiB/s of uncompressed data through the K timed steps above (H2D + D2H inside the timed region; for N > 1 also
              the NCCL gather of the compressed blocks to rank 0, bzip3_b200/sharding.py).  `ms_per_step` is this loop's.
   value      the same round trip with the inputs already resident in HBM (bz3_b200_encode_resident_many /
-             bz3_b200_decode_resident_many), a 1 + 2 step side loop: the two differ by the PCIe copies only (< 0.1 %).
+             bz3_b200_decode_resident_many), a side loop of W warm-up + K timed steps: the two differ by the PCIe copies
+             only (< 0.1 %).
   headline_b256   BASELINE.json's metric configuration (1 GiB synthetic source corpus, -b 256, 4 blocks of 256 MiB per
              GPU): 1 warm-up + 1 timed e2e step, block 0 compared with the reference encoder, the reference's pthread
              path timed on the same bytes.  Skipped with --no-headline or when the run is already late.
@@ -257,6 +258,21 @@ def run_reference_arm(args, rank, world):
 
 
 # ------------------------------------------------------------------------------------------- B200 arm
+DUMP_SAMPLE = 7_500_000   # float32 values per byte array written by --dump-outputs: 60 MB for the two, under 64 MB
+
+
+def dump_outputs(path, comp_sizes, compressed, decoded):
+    """--dump-outputs: what the last timed step handed back to its caller, as DIR/<name>.npy.  Bytes are stored as
+    float32 (exact).  A byte array longer than DUMP_SAMPLE is replaced by its values at DUMP_SAMPLE sorted indices drawn
+    from a fixed seed, so two builds that return arrays of the same length are sampled at the same places."""
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "compressed_sizes.npy"), np.asarray(comp_sizes, np.float64))
+    for name, a in (("compressed_bytes", compressed), ("decoded_bytes", decoded)):
+        if a.size > DUMP_SAMPLE:
+            a = a[np.sort(np.random.default_rng(2026).integers(0, a.size, DUMP_SAMPLE))]
+        np.save(os.path.join(path, name + ".npy"), a.astype(np.float32))
+
+
 class Job:
     """The rank's blocks, one bz3_state per block, pinned host buffers for the ABI path."""
 
@@ -329,13 +345,16 @@ def run_b200_arm(args, rank, world, local_rank):
             dist.barrier()
         torch.cuda.synchronize()
 
-    def e2e_step(job):
-        """encode + (N > 1: ordered gather of the compressed blocks to rank 0) + decode through the ABI on host buffers"""
+    def e2e_step(job, keep=None):
+        """encode + (N > 1: ordered gather of the compressed blocks to rank 0) + decode through the ABI on host buffers;
+        `keep` (a list) receives the compressed blocks, which the decode overwrites in place"""
         job.stage_host()
         flush.fill_(1)
         barrier()
         ev[0].record()
         csz = job.encode_abi()
+        if keep is not None:
+            keep.extend(p[:c].numpy().copy() for p, c in zip(job.pinned, job.comp))
         if dist:  # the path's only exchange (SURVEY.md 8e): sizes by all_gather, padded payloads gathered to rank 0
             mine = {rank + k * world: job.pinned[k][:c].numpy() for k, c in enumerate(job.comp)}
             sharding.gather_compressed(mine, job.nb * world, rank, world, dist)
@@ -373,12 +392,12 @@ def run_b200_arm(args, rank, world, local_rank):
     gate = gated_roundtrip(job)
     gate_comp = list(job.comp)
 
-    # ---------------- device-resident side loop: 1 warm-up + 2 timed steps
+    # ---------------- device-resident side loop: W warm-up + K timed steps
     sizes = (C.c_int32 * nb)(*[len(b) for b in job.blocks])
     enc_sizes = (C.c_int32 * nb)()
     dec_res = (C.c_int32 * nb)()
     res_ms = []
-    for i in range(3):
+    for i in range(args.warmup + args.steps):
         for s, b in zip(job.states, job.blocks):
             assert L.bz3_b200_upload(s.handle, refs.ptr(b), len(b)) == 0
         flush.fill_(1)
@@ -390,7 +409,7 @@ def run_b200_arm(args, rank, world, local_rank):
         ev[2].record()
         torch.cuda.synchronize()
         assert list(dec_res) == [len(b) for b in job.blocks], list(dec_res)
-        if i >= 1:
+        if i >= args.warmup:
             res_ms.append((ev[0].elapsed_time(ev[1]), ev[1].elapsed_time(ev[2])))
     res_enc = reduce_max(sum(t[0] for t in res_ms) / len(res_ms))
     res_dec = reduce_max(sum(t[1] for t in res_ms) / len(res_ms))
@@ -405,8 +424,12 @@ def run_b200_arm(args, rank, world, local_rank):
     sampler = ClockSampler(local_rank)
     if rank == 0:
         sampler.start()
-    e2e_ms = [e2e_step(job) for _ in range(args.steps)]
+    kept = [] if args.dump_outputs and rank == 0 else None
+    e2e_ms = [e2e_step(job, kept if i == args.steps - 1 else None) for i in range(args.steps)]
     clocks = sampler.stop() if rank == 0 else None
+    if kept is not None:
+        dump_outputs(args.dump_outputs, job.comp, np.concatenate(kept),
+                     np.concatenate([p[:len(b)].numpy() for p, b in zip(job.pinned, job.blocks)]))
     e2e_step_ms = reduce_max(sum(e2e_ms)) / args.steps
     e2e_val = job_bytes / MIB / (e2e_step_ms / 1e3)
     launches = sum(s.launches() for s in job.states)
@@ -520,8 +543,8 @@ def run_b200_arm(args, rank, world, local_rank):
                        "bytes_per_gpu": total, "parallelism": f"blocks sharded {world} way(s), one stream per block",
                        "l2": "256 MiB flush buffer written before every timed step; block buffers + shared stage workspaces >> 126 MB L2",
                        "timed_loop": "the K steps are the e2e path (reference ABI, pinned host buffers); `value` is the device-resident "
-                                     "round trip from a 1 + 2 step side loop (the two differ by the PCIe copies only)",
-                       "value_steps": 2, "value_ms_per_step": round(res_step, 3),
+                                     "round trip from a side loop of W + K steps (the two differ by the PCIe copies only)",
+                       "value_steps": args.steps, "value_ms_per_step": round(res_step, 3),
                        "bit_exact": gate,
                        "hbm_bytes": {"per_block_state": dev_state_bytes, "shared_stage_workspaces": dev_ws_bytes,
                                      "stage_workspaces": int(os.environ.get("BZ3_B200_ARENAS", "2"))},
@@ -592,7 +615,12 @@ def main():
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--workload", default=os.environ.get("BZ3_BENCH_WORKLOAD", "zipf100m_b16"), choices=sorted(WORKLOADS))
     ap.add_argument("--no-headline", action="store_true", help="skip the 256 MiB-block sub-record")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned (rank 0's compressed block sizes, compressed bytes and "
+                         "decoded bytes) to DIR/<name>.npy; the compressed blocks are copied aside inside that step")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

@@ -1,6 +1,9 @@
-"""ctypes access to the CPU oracle (oracle/_build/liboracle.so) and, when it was built, to the
-unmodified reference (oracle/_ref/*.so).  Test infrastructure only."""
+"""ctypes access to the CPU oracle (oracle/_build/liboracle.so), to the answers of the unmodified reference
+stored under tests/golden, and, when it was built, to the reference itself (oracle/_ref/*.so).  Test
+infrastructure only."""
 import ctypes as C
+import hashlib
+import json
 import os
 import subprocess
 
@@ -12,9 +15,33 @@ REF_SO = os.path.join(ROOT, "oracle", "_ref", "libbz3_ref.so")
 REF_STAGES_SO = os.path.join(ROOT, "oracle", "_ref", "libbz3_ref_stages.so")
 REF_CLI = os.path.join(ROOT, "oracle", "_ref", "bzip3_ref")
 GOLDEN = os.path.join(ROOT, "tests", "golden")
+ANSWERS = os.path.join(GOLDEN, "reference_answers.json")
 
 u8p = C.POINTER(C.c_uint8)
 i32p = C.POINTER(C.c_int32)
+
+
+def digest(b) -> str:
+    """Content digest of a byte string in the stored reference answers: the first 16 hex digits of its SHA-256."""
+    return hashlib.sha256(bytes(b)).hexdigest()[:16]
+
+
+_answers = None
+
+
+def reference_answer(key):
+    """What the unmodified reference computed for `key`, as written by tests/golden/make_reference_answers.py."""
+    global _answers
+    if _answers is None:
+        with open(ANSWERS) as f:
+            _answers = json.load(f)
+    return _answers[key]
+
+
+def check_answer(key, got):
+    """`got` (ints, strings and lists of them) must equal the stored reference answer for `key`."""
+    got, want = json.loads(json.dumps(got)), reference_answer(key)
+    assert got == want, f"{key}: {got} differs from the reference's {want}"
 
 
 def build_oracle():

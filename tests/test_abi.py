@@ -1,8 +1,9 @@
 """CPU-only: the CUDA library builds, loads without a GPU, exports every symbol include/*.h declares,
 and refuses to work (instead of falling back to a CPU path) when no device is present."""
-import ctypes as C
 import os
 import re
+import subprocess
+import sys
 
 import pytest
 
@@ -48,20 +49,26 @@ def test_pure_host_helpers(L):
     b = 65 * 1024 + 65 * 1024 // 50 + 32
     assert L.bz3_min_memory_needed(65 * 1024) == 48 + 149024 + b + 4 * (b + 128) + 4 * (1 << 18)
     from tests import refs
-    if refs.have_ref():   # the compiled reference itself, when it is there
-        R = refs.ref()
-        R.bz3_min_memory_needed.restype = C.c_size_t
-        R.bz3_min_memory_needed.argtypes = [C.c_int32]
-        for bs in (1000, 65 * 1024, 1 << 20, 16 << 20, 256 << 20, 511 << 20, (511 << 20) + 1):
-            assert L.bz3_min_memory_needed(bs) == R.bz3_min_memory_needed(bs), bs
+    # the reference's figures
+    refs.check_answer("min_memory_needed", [L.bz3_min_memory_needed(bs) for bs in MIN_MEMORY_BLOCK_SIZES])
     assert L.bz3_new(1000) is None  # block size out of range never needs a device
 
 
+MIN_MEMORY_BLOCK_SIZES = (1000, 65 * 1024, 1 << 20, 16 << 20, 256 << 20, 511 << 20, (511 << 20) + 1)
+
+
 def test_no_device_means_failure_not_fallback(L):
-    import torch
-    if torch.cuda.is_available():
-        pytest.skip("a GPU is present")
-    assert L.bz3_b200_device_count() == 0
-    assert L.bz3_new(1 << 20) is None
-    with pytest.raises(bzip3_b200.Bz3Error):
-        bzip3_b200.Bz3State(1 << 20)
+    """In a child process that sees no device (CUDA_VISIBLE_DEVICES empty), so that it runs on GPU machines too."""
+    script = ("import sys\n"
+              "sys.path.insert(0, %r)\n"
+              "import bzip3_b200\n"
+              "L = bzip3_b200.lib()\n"
+              "assert L.bz3_b200_device_count() == 0\n"
+              "assert L.bz3_new(1 << 20) is None\n"
+              "try:\n"
+              "    bzip3_b200.Bz3State(1 << 20)\n"
+              "except bzip3_b200.Bz3Error:\n"
+              "    print('REFUSED')\n" % ROOT)
+    env = dict(os.environ, CUDA_VISIBLE_DEVICES="")
+    r = subprocess.run([sys.executable, "-c", script], env=env, capture_output=True, text=True, timeout=300)
+    assert r.returncode == 0 and "REFUSED" in r.stdout, r.stdout + r.stderr

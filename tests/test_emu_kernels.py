@@ -105,6 +105,21 @@ def test_cm_decode_exhausted_streams():
     kernel's shortcuts (one renormalisation test per byte, range < 2^24 as the cheap pre-test) are switched off from
     there on, so truncated and garbage payloads decode exactly like the reference -- for as long as the caller asks."""
     E, O = emu(), refs.oracle()
+    n, payloads = exhausted_payloads()
+    pins = refs.reference_answer("cm_exhausted")   # the oracle itself is pinned on the reference for these payloads
+    assert len(pins) == len(payloads)
+    for (buf, insize), pin in zip(payloads, pins):
+        want = np.zeros(n + 8, np.uint8)
+        got = np.zeros(n + 8, np.uint8)
+        O.orc_cm_decode(refs.ptr(buf), insize, refs.ptr(want), n)
+        assert refs.digest(want[:n]) == pin, insize
+        assert E.emu_cm_decode(refs.ptr(buf), insize, refs.ptr(got), n) == 0
+        assert bytes(got[:n]) == bytes(want[:n]), insize
+
+
+def exhausted_payloads():
+    """(n, [(payload, insize)]): a CM payload cut short at many places, and garbage of a few bytes, decoded to n bytes."""
+    O = refs.oracle()
     rng = np.random.default_rng(31337)
     data = CM_CASES[CM_IDS.index("bwt_zipf_12k")][1][:1500]
     n = len(data)
@@ -116,16 +131,7 @@ def test_cm_decode_exhausted_streams():
         m = int(rng.integers(1, 40))
         g[:m] = rng.integers(0, 256, m, dtype=np.uint8) if k % 3 else np.full(m, 255 * (k % 2), np.uint8)
         payloads.append((g, m))
-    for buf, insize in payloads:
-        want = np.zeros(n + 8, np.uint8)
-        got = np.zeros(n + 8, np.uint8)
-        O.orc_cm_decode(refs.ptr(buf), insize, refs.ptr(want), n)
-        if refs.have_ref():   # the oracle itself is pinned on the reference for these payloads
-            pin = np.zeros(n + 8, np.uint8)
-            refs.ref_stages().ref_cm_decode(refs.ptr(buf.copy()), insize, refs.ptr(pin), n)
-            assert bytes(pin[:n]) == bytes(want[:n]), insize
-        assert E.emu_cm_decode(refs.ptr(buf), insize, refs.ptr(got), n) == 0
-        assert bytes(got[:n]) == bytes(want[:n]), insize
+    return n, payloads
 
 
 @pytest.mark.parametrize("schedule", [1, 2])

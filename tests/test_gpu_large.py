@@ -1,8 +1,8 @@
-"""Large blocks on the GPU against the compiled reference (oracle/_ref): the encoded block must equal the reference's
-bz3_encode_block output byte for byte and decode both ways, up to the metric's block size (256 MiB, BASELINE.json
-configs[2]) and the format's maximum (511 MiB, configs[4]; src/libbz3.c:536); plus the batch API at the benchmark's
-block size.  The reference's side of the two big cases runs on a host thread while the GPU works (about a minute each)."""
-import os
+"""Large blocks on the GPU against the reference: the encoded block must equal the reference's bz3_encode_block output
+byte for byte (its size and digest, tests/golden/reference_answers.json) and decode, up to the metric's block size
+(256 MiB, BASELINE.json configs[2]) and the format's maximum (511 MiB, configs[4]; src/libbz3.c:536); plus the batch API
+at the benchmark's block size.  The reference decodes each of its blocks to the input where the answers were made, so
+a block equal to the reference's decodes there too."""
 import struct
 
 import numpy as np
@@ -14,34 +14,40 @@ from tests import refs
 
 pytestmark = pytest.mark.gpu
 
+# the single blocks compared with the reference's: answer key -> a function making their bytes
+BLOCKS = {
+    "large/source_64mib": lambda: synth.source_corpus(64 << 20, seed=1234 + 64),
+    "large/mixed_32mib": lambda: synth.mixed(32 << 20, seed=1234 + 32, segment=4 << 20),
+    "large/source_256mib": lambda: synth.source_corpus(256 << 20, seed=synth.SEED_SOURCE),
+    "large/log_511mib": lambda: synth.log_stream(511 << 20, seed=synth.SEED_LOG),
+}
 
-def roundtrip(block_mib, gen, check_reference):
-    n = block_mib << 20
-    data = gen(n, seed=1234 + block_mib)
+
+def roundtrip(key):
+    data = BLOCKS[key]()
+    n = len(data)
     with bzip3_b200.Bz3State(n) as s:
         enc, r = s.encode_block(data.tobytes())
         assert r > 0 and s.last_error == 0
         crc, idx, model = struct.unpack("<IiB", enc[:9])
         assert crc == refs.oracle().orc_crc32(1, refs.ptr(data), n)
         assert 1 <= idx <= n
-        if check_reference and refs.have_ref():
-            want = refs.api_encode_block(refs.ref(), data.tobytes(), n)[0]
-            assert want == enc, "differs from the reference encoder"
+        refs.check_answer(key, [r, s.last_error, refs.digest(enc)])
         dec, r2 = s.decode_block(enc, n)
         assert r2 == n and s.last_error == 0 and dec == data.tobytes()
 
 
 def test_roundtrip_64mib_source_block():
-    roundtrip(64, synth.source_corpus, check_reference=True)
+    roundtrip("large/source_64mib")
 
 
 def test_roundtrip_32mib_mixed_block_with_incompressible_segments():
-    roundtrip(32, lambda n, seed: synth.mixed(n, seed=seed, segment=4 << 20), check_reference=True)
+    roundtrip("large/mixed_32mib")
 
 
 def test_batch_of_16mib_blocks_matches_reference():
     bs = 16 << 20
-    datas = [synth.zipf_text(bs, seed=77).tobytes(), synth.log_stream(bs // 2, seed=78).tobytes()]
+    datas = batch_16mib_data()
     states = [bzip3_b200.Bz3State(bs) for _ in datas]
     try:
         bufs = []
@@ -51,15 +57,18 @@ def test_batch_of_16mib_blocks_matches_reference():
             bufs.append(b)
         sizes = bzip3_b200.encode_blocks(states, bufs, [len(d) for d in datas])
         assert all(s.last_error == 0 for s in states)
-        if refs.have_ref():
-            for d, b, sz in zip(datas, bufs, sizes):
-                assert refs.api_encode_block(refs.ref(), d, bs)[0] == bytes(b[:sz])
+        refs.check_answer("large/batch_16mib", [[sz, refs.digest(b[:sz])] for b, sz in zip(bufs, sizes)])
         bzip3_b200.decode_blocks(states, bufs, [len(b) for b in bufs], sizes, [len(d) for d in datas])
         for d, b, s in zip(datas, bufs, states):
             assert s.last_error == 0 and bytes(b[:len(d)]) == d
     finally:
         for s in states:
             s.close()
+
+
+def batch_16mib_data():
+    bs = 16 << 20
+    return [synth.zipf_text(bs, seed=77).tobytes(), synth.log_stream(bs // 2, seed=78).tobytes()]
 
 
 def test_many_blocks_of_mixed_sizes_at_once():
@@ -94,60 +103,28 @@ def test_many_blocks_of_mixed_sizes_at_once():
             s.close()
 
 
-def _against_reference_big(n, data):
-    """encode on the GPU and with the reference at the same time, compare, decode both ways"""
-    import threading
-    assert refs.have_ref(), "oracle/_ref is missing: run `make -C oracle ref` where /root/reference exists"
-    R = refs.ref()
+def _against_reference_big(key):
+    """encode on the GPU, compare with the reference's block, decode"""
+    data = BLOCKS[key]()
+    n = len(data)
+    L = bzip3_b200.lib()
     cap = refs.bound(n) + 64
-    rbuf = np.zeros(cap, np.uint8)
-    rbuf[:n] = data
-    rst = R.bz3_new(n)
-    assert rst
-    rres = {}
-
-    def ref_side():
-        rres["size"] = R.bz3_encode_block(rst, refs.ptr(rbuf), n)
-        rres["err"] = R.bz3_last_error(rst)
-
-    th = threading.Thread(target=ref_side)
-    th.start()
     gbuf = np.zeros(cap, np.uint8)
     gbuf[:n] = data
-    L = bzip3_b200.lib()
-    try:
-        with bzip3_b200.Bz3State(n) as s:
-            r = L.bz3_encode_block(s.handle, refs.ptr(gbuf), n)
-            assert r > 0 and s.last_error == 0, (r, s.last_error)
-            th.join()
-            assert rres["err"] == 0 and rres["size"] == r, (rres, r)
-            assert np.array_equal(gbuf[:r], rbuf[:r]), "block differs from the reference's bz3_encode_block output"
-            # the reference decodes the GPU's block (host thread) while the GPU decodes the reference's
-            def ref_decode():
-                rres["dec"] = R.bz3_decode_block(rst, refs.ptr(rbuf), cap, r, n)
-                rres["derr"] = R.bz3_last_error(rst)
-            rbuf[:r] = gbuf[:r]
-            th2 = threading.Thread(target=ref_decode)
-            th2.start()
-            r2 = L.bz3_decode_block(s.handle, refs.ptr(gbuf), cap, r, n)
-            assert r2 == n and s.last_error == 0, (r2, s.last_error)
-            assert np.array_equal(gbuf[:n], data), "GPU decode of the block differs from the input"
-            th2.join()
-            assert rres["dec"] == n and rres["derr"] == 0, rres
-            assert np.array_equal(rbuf[:n], data), "the reference decodes the GPU's block to something else"
-    finally:
-        if th.is_alive():
-            th.join()
-        R.bz3_free(rst)
+    with bzip3_b200.Bz3State(n) as s:
+        r = L.bz3_encode_block(s.handle, refs.ptr(gbuf), n)
+        assert r > 0 and s.last_error == 0, (r, s.last_error)
+        refs.check_answer(key, [r, s.last_error, refs.digest(gbuf[:r])])
+        r2 = L.bz3_decode_block(s.handle, refs.ptr(gbuf), cap, r, n)
+        assert r2 == n and s.last_error == 0, (r2, s.last_error)
+        assert np.array_equal(gbuf[:n], data), "GPU decode of the block differs from the input"
 
 
 def test_256mib_block_equals_the_reference():
     """the metric's block size: one 256 MiB block of the synthetic source corpus (BASELINE.json configs[2])"""
-    n = 256 << 20
-    _against_reference_big(n, synth.source_corpus(n, seed=synth.SEED_SOURCE))
+    _against_reference_big("large/source_256mib")
 
 
 def test_511mib_block_equals_the_reference():
     """the largest block the format allows (src/libbz3.c:536): 511 MiB of the synthetic log stream (configs[4])"""
-    n = 511 << 20
-    _against_reference_big(n, synth.log_stream(n, seed=synth.SEED_LOG))
+    _against_reference_big("large/log_511mib")

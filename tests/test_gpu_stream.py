@@ -1,6 +1,6 @@
 """The container front end with the deep block queue (bz3_b200_encode_fd / bz3_b200_decode_fd, csrc/stream.h) on the GPU:
 more blocks than queue slots, several blocks in flight, bytes compared with the reference tool's container built around
-the oracle's blocks (and with the reference binary where oracle/_ref travelled along)."""
+the oracle's blocks (and with what the reference binary wrote, tests/golden/reference_answers.json)."""
 import ctypes as C
 import os
 import struct
@@ -25,10 +25,14 @@ def container(data, bs):
     return bytes(out)
 
 
+def corpus_data():
+    return (synth.zipf_text(2_300_000, seed=21).tobytes() + bytes(300_000) + synth.log_stream(1_900_000, seed=22).tobytes()
+            + synth.source_corpus(1_200_000, seed=23).tobytes() + b"end")
+
+
 @pytest.fixture(scope="module")
 def corpus():
-    data = (synth.zipf_text(2_300_000, seed=21).tobytes() + bytes(300_000) + synth.log_stream(1_900_000, seed=22).tobytes()
-            + synth.source_corpus(1_200_000, seed=23).tobytes() + b"end")
+    data = corpus_data()
     return data, container(data, BS)
 
 
@@ -85,10 +89,8 @@ def test_command_line_tool(tmp_path, corpus):
     r = subprocess.run([cli, "-e", "-b", "1", "-j", "5"], input=data, capture_output=True, timeout=600)
     assert r.returncode == 0, r.stderr
     assert r.stdout == want
-    if os.path.exists(refs.REF_CLI):
-        ref = subprocess.run([refs.REF_CLI, "-e", "-b", "1", "-j", "4"], input=data, capture_output=True, check=True, timeout=600).stdout
-        assert r.stdout == ref
-        assert subprocess.run([refs.REF_CLI, "-d"], input=r.stdout, capture_output=True, check=True, timeout=600).stdout == data
+    # what `bzip3 -e -b 1 -j 4` writes for the same input; the reference decodes that file to the input
+    refs.check_answer("cli/stream_corpus_b1", [len(r.stdout), refs.digest(r.stdout)])
     r = subprocess.run([cli, "-d", "-j", "3"], input=want, capture_output=True, timeout=600)
     assert r.returncode == 0 and r.stdout == data
 

@@ -1,12 +1,15 @@
 """Pins the CPU oracle (oracle/bz3_oracle.c) against
   (1) the reference's golden vector  examples/shakespeare.txt(.bz3)  (Makefile.am:81-83),
   (2) known answers computed by the compiled reference (SURVEY.md 8c / BASELINE.md section 2),
-  (3) the unmodified reference compiled from /root/reference into oracle/_ref (when present),
-stage by stage and block by block.  CPU only."""
+  (3) what the unmodified reference computes for the same inputs, stage by stage and block by block
+      (tests/golden/reference_answers.json, written by tests/golden/make_reference_answers.py through the
+      *_answer functions below).
+CPU only."""
 import ctypes as C
 import hashlib
 import os
 import struct
+from types import SimpleNamespace
 
 import numpy as np
 import pytest
@@ -15,9 +18,15 @@ from bzip3_b200 import synth
 from tests import refs
 
 O = refs.oracle()
-needs_ref = pytest.mark.skipif(not refs.have_ref(), reason="oracle/_ref not built (no /root/reference here)")
 CASES = synth.edge_cases()
 IDS = [c[0] for c in CASES]
+# the stage and block functions of the oracle; the reference's, with the same calling convention, are in
+# tests/golden/make_reference_answers.py
+ORACLE_STAGES = SimpleNamespace(crc=O.orc_crc32, mrle_encode=O.orc_mrle_encode, mrle_decode=O.orc_mrle_decode,
+                                lzp_encode=O.orc_lzp_encode, lzp_decode=O.orc_lzp_decode, bwt=O.orc_bwt,
+                                unbwt=O.orc_unbwt, cm_encode=O.orc_cm_encode, cm_decode=O.orc_cm_decode)
+ORACLE_BLOCKS = SimpleNamespace(encode=refs.oracle_encode_block, decode=refs.oracle_decode_block)
+HOSTILE = ["raw63", "coded65_text", "zeros_4k", "random_10k", "repeat_block_5000x20", "long_runs", "zipf_200k"]
 
 
 def arr(b):
@@ -83,142 +92,133 @@ def test_seed_files_roundtrip(name):
 
 
 # ------------------------------------------------------------------ stage-level differential vs the reference
-@needs_ref
-@pytest.mark.parametrize("name,data", CASES, ids=IDS)
-def test_stage_crc(name, data):
-    R = refs.ref_stages()
+# Each *_answer function runs one comparison on one implementation and returns what it saw: return values and digests
+# of the bytes written.  The tests take the oracle's; the stored answers are the reference's, through the same function.
+def crc_answer(S, data):
     a = arr(data)
-    assert O.orc_crc32(1, refs.ptr(a), len(a)) == R.ref_crc32(1, refs.ptr(a), len(a))
+    return S.crc(1, refs.ptr(a), len(a))
 
 
-@needs_ref
-@pytest.mark.parametrize("name,data", CASES, ids=IDS)
-def test_stage_mrle(name, data):
-    R = refs.ref_stages()
+def mrle_answer(S, data):
+    """mRLE encode, then decodes of the whole encoding and of truncated ones: the failure flag and the bytes produced
+    must agree too."""
     a = arr(data)
     n = len(a)
-    o1 = np.zeros(2 * n + 64, np.uint8)
-    o2 = np.zeros(2 * n + 64, np.uint8)
-    r1 = O.orc_mrle_encode(refs.ptr(a), n, refs.ptr(o1))
-    r2 = R.ref_mrlec(refs.ptr(a.copy()), n, refs.ptr(o2))
-    assert r1 == r2 and bytes(o1[:r1]) == bytes(o2[:r2])
-    d1 = np.zeros(n + 8, np.uint8)
-    d2 = np.zeros(n + 8, np.uint8)
-    assert O.orc_mrle_decode(refs.ptr(o1), refs.ptr(d1), n, r1) == R.ref_mrled(refs.ptr(o2), refs.ptr(d2), n, r2) == 0
-    assert bytes(d1[:n]) == bytes(d2[:n]) == bytes(a)
-    # truncated / wrong-length inputs must agree on the failure flag and on the bytes produced
-    for cut in (r1 - 1, r1 // 2, 33, 32, 31):
+    o = np.zeros(2 * n + 64, np.uint8)
+    r = S.mrle_encode(refs.ptr(a.copy()), n, refs.ptr(o))
+    out = [r, refs.digest(o[:r])]
+    for cut in (r, r - 1, r // 2, 33, 32, 31):
         if cut < 0:
             continue
-        d1[:] = 0
-        d2[:] = 0
-        e1 = O.orc_mrle_decode(refs.ptr(o1), refs.ptr(d1), n, cut)
-        e2 = R.ref_mrled(refs.ptr(o2), refs.ptr(d2), n, cut)
-        assert e1 == e2 and bytes(d1) == bytes(d2)
+        d = np.zeros(n + 8, np.uint8)
+        e = S.mrle_decode(refs.ptr(o), refs.ptr(d), n, cut)
+        out.append([cut, e, refs.digest(d[:n] if cut == r else d)])
+    return out
 
 
-@needs_ref
-@pytest.mark.parametrize("name,data", CASES, ids=IDS)
-def test_stage_lzp(name, data):
-    R = refs.ref_stages()
+def lzp_answer(S, data):
+    """LZP encode, then decodes of the whole encoding and of truncated ones with the same table."""
     a = arr(data)
     n = len(a)
     pad = np.zeros(n + 64, np.uint8)
     pad[:n] = a
-    o1 = np.zeros(n + 64, np.uint8)
-    o2 = np.zeros(n + 64, np.uint8)
-    lut1 = np.zeros(1 << 18, np.int32)
-    lut2 = np.zeros(1 << 18, np.int32)
-    l1 = lut1.ctypes.data_as(refs.i32p)
-    l2 = lut2.ctypes.data_as(refs.i32p)
-    r1 = O.orc_lzp_encode(refs.ptr(pad), n, refs.ptr(o1), l1)
-    r2 = R.ref_lzp_compress(refs.ptr(pad), refs.ptr(o2), n, l2)
-    assert r1 == r2
-    if r1 > 0:
-        assert bytes(o1[:r1]) == bytes(o2[:r2])
+    o = np.zeros(n + 64, np.uint8)
+    lut = np.zeros(1 << 18, np.int32)
+    lp = lut.ctypes.data_as(refs.i32p)
+    r = S.lzp_encode(refs.ptr(pad), n, refs.ptr(o), lp)
+    out = [r]
+    if r > 0:
+        out.append(refs.digest(o[:r]))
         cap = refs.bound(n) + 64
-        d1 = np.zeros(cap, np.uint8)
-        d2 = np.zeros(cap, np.uint8)
-        s1 = O.orc_lzp_decode(refs.ptr(o1), r1, refs.ptr(d1), refs.bound(n), l1)
-        s2 = R.ref_lzp_decompress(refs.ptr(o2), refs.ptr(d2), r2, refs.bound(n), l2)
-        assert s1 == s2 == n and bytes(d1[:n]) == bytes(a)
-        for cut in (r1 - 1, r1 - 2, r1 // 2, 5, 4, 3):
+        for cut in (r, r - 1, r - 2, r // 2, 5, 4, 3):
             if cut < 0:
                 continue
-            d1[:] = 0
-            d2[:] = 0
-            s1 = O.orc_lzp_decode(refs.ptr(o1), cut, refs.ptr(d1), refs.bound(n), l1)
-            s2 = R.ref_lzp_decompress(refs.ptr(o2), refs.ptr(d2), cut, refs.bound(n), l2)
-            assert s1 == s2
-            if s1 > 0:
-                assert bytes(d1[:s1]) == bytes(d2[:s2])
+            d = np.zeros(cap, np.uint8)
+            s = S.lzp_decode(refs.ptr(o), cut, refs.ptr(d), refs.bound(n), lp)
+            out.append([cut, s, refs.digest(d[:s]) if s > 0 else None])
+    return out
 
 
-@needs_ref
+def bwt_answer(S, data):
+    """BWT, its inverse, and the inverse with primary indices out of range."""
+    a = arr(data)
+    n = len(a)
+    u = np.zeros(n + 8, np.uint8)
+    i = S.bwt(refs.ptr(a), refs.ptr(u), n)
+    t = np.zeros(n + 8, np.uint8)
+    out = [i, refs.digest(u[:n]), S.unbwt(refs.ptr(u), refs.ptr(t), n, i), refs.digest(t[:n])]
+    if n >= 2:
+        out.append([S.unbwt(refs.ptr(u), refs.ptr(t), n, bad) for bad in (0, -3, n + 1)])
+    return out
+
+
+def cm_answer(S, data):
+    """CM encode, then decodes of the whole payload and of truncated ones (read as 0xFF.. like read_in)."""
+    a = arr(data)
+    n = len(a)
+    o = np.zeros(2 * n + 64, np.uint8)
+    r = S.cm_encode(refs.ptr(a.copy()), n, refs.ptr(o))
+    out = [r, refs.digest(o[:r])]
+    for insize in (r, max(r - 3, 0), r // 2, 0):
+        d = np.zeros(n + 8, np.uint8)
+        S.cm_decode(refs.ptr(o), insize, refs.ptr(d), n)
+        out.append([insize, refs.digest(d)])
+    return out
+
+
+@pytest.mark.parametrize("name,data", CASES, ids=IDS)
+def test_stage_crc(name, data):
+    refs.check_answer(f"stage_crc/{name}", crc_answer(ORACLE_STAGES, data))
+
+
+@pytest.mark.parametrize("name,data", CASES, ids=IDS)
+def test_stage_mrle(name, data):
+    got = mrle_answer(ORACLE_STAGES, data)
+    refs.check_answer(f"stage_mrle/{name}", got)
+    assert got[2][1:] == [0, refs.digest(data)]
+
+
+@pytest.mark.parametrize("name,data", CASES, ids=IDS)
+def test_stage_lzp(name, data):
+    got = lzp_answer(ORACLE_STAGES, data)
+    refs.check_answer(f"stage_lzp/{name}", got)
+    if got[0] > 0:
+        assert got[2][1:] == [len(data), refs.digest(data)]
+
+
 @pytest.mark.parametrize("name,data", CASES, ids=IDS)
 def test_stage_bwt(name, data):
-    R = refs.ref_stages()
-    a = arr(data)
-    n = len(a)
-    u1 = np.zeros(n + 8, np.uint8)
-    u2 = np.zeros(n + 8, np.uint8)
-    A = np.zeros(n + 256, np.int32)
-    i1 = O.orc_bwt(refs.ptr(a), refs.ptr(u1), n)
-    i2 = R.ref_bwt(refs.ptr(a), refs.ptr(u2), A.ctypes.data_as(refs.i32p), n)
-    assert i1 == i2 and bytes(u1[:n]) == bytes(u2[:n])
-    t1 = np.zeros(n + 8, np.uint8)
-    t2 = np.zeros(n + 8, np.uint8)
-    A[:] = 0
-    assert O.orc_unbwt(refs.ptr(u1), refs.ptr(t1), n, i1) == R.ref_unbwt(refs.ptr(u2), refs.ptr(t2),
-                                                                         A.ctypes.data_as(refs.i32p), n, i2) == 0
-    assert bytes(t1[:n]) == bytes(t2[:n]) == bytes(a)
-    for bad in (0, -3, n + 1):
-        if n >= 2:
-            A[:] = 0
-            assert O.orc_unbwt(refs.ptr(u1), refs.ptr(t1), n, bad) == R.ref_unbwt(
-                refs.ptr(u2), refs.ptr(t2), A.ctypes.data_as(refs.i32p), n, bad) == -1
+    got = bwt_answer(ORACLE_STAGES, data)
+    refs.check_answer(f"stage_bwt/{name}", got)
+    assert got[2:4] == [0, refs.digest(data)]
 
 
-@needs_ref
 @pytest.mark.parametrize("name,data", CASES, ids=IDS)
 def test_stage_cm(name, data):
-    R = refs.ref_stages()
-    a = arr(data)
-    n = len(a)
-    o1 = np.zeros(2 * n + 64, np.uint8)
-    o2 = np.zeros(2 * n + 64, np.uint8)
-    r1 = O.orc_cm_encode(refs.ptr(a), n, refs.ptr(o1))
-    r2 = R.ref_cm_encode(refs.ptr(a.copy()), n, refs.ptr(o2))
-    assert r1 == r2 and bytes(o1[:r1]) == bytes(o2[:r2])
-    for insize in (r1, max(r1 - 3, 0), r1 // 2, 0):  # truncated payloads read as 0xFF.. like read_in
-        d1 = np.zeros(n + 8, np.uint8)
-        d2 = np.zeros(n + 8, np.uint8)
-        O.orc_cm_decode(refs.ptr(o1), insize, refs.ptr(d1), n)
-        R.ref_cm_decode(refs.ptr(o2), insize, refs.ptr(d2), n)
-        assert bytes(d1) == bytes(d2)
-        if insize == r1:
-            assert bytes(d1[:n]) == bytes(a)
+    got = cm_answer(ORACLE_STAGES, data)
+    refs.check_answer(f"stage_cm/{name}", got)
+    assert got[2][1] == refs.digest(data + bytes(8))
 
 
 # ------------------------------------------------------------------ block-level differential
-@needs_ref
+def block_answer(B, data):
+    bs = max(65 * 1024, len(data))
+    enc, r, e = B.encode(data, bs)
+    dec, d, de = B.decode(enc, len(data), bs)
+    return [r, e, refs.digest(enc), d, de, refs.digest(dec)]
+
+
 @pytest.mark.parametrize("name,data", CASES, ids=IDS)
 def test_block_encode_decode_vs_reference(name, data):
-    L = refs.ref()
-    bs = max(65 * 1024, len(data))
-    enc_r, r_r, e_r = refs.api_encode_block(L, data, bs)
-    enc_o, r_o, e_o = refs.oracle_encode_block(data, bs)
-    assert (r_r, e_r) == (r_o, e_o) and enc_r == enc_o
-    dec_r, d_r, de_r = refs.api_decode_block(L, enc_r, len(data), bs)
-    dec_o, d_o, de_o = refs.oracle_decode_block(enc_o, len(data), bs)
-    assert (d_r, de_r) == (d_o, de_o) == (len(data), 0) and dec_r == dec_o == data
+    got = block_answer(ORACLE_BLOCKS, data)
+    refs.check_answer(f"block/{name}", got)
+    assert got[3:] == [len(data), 0, refs.digest(data)]
 
 
-@needs_ref
 def test_block_too_big():
-    L = refs.ref()
-    data = bytes(70000)
-    assert refs.api_encode_block(L, data, 65 * 1024)[1:] == refs.oracle_encode_block(data, 65 * 1024)[1:] == (-1, -6)
+    got = list(refs.oracle_encode_block(bytes(70000), 65 * 1024)[1:])
+    refs.check_answer("block_too_big", got)
+    assert got == [-1, -6]
 
 
 def hostile_variants(enc, osz, bs, rng):
@@ -244,31 +244,40 @@ def hostile_variants(enc, osz, bs, rng):
     return out
 
 
-@needs_ref
-@pytest.mark.parametrize("name", ["raw63", "coded65_text", "zeros_4k", "random_10k", "repeat_block_5000x20",
-                                  "long_runs", "zipf_200k"])
-def test_hostile_decode_error_parity(name):
-    L = refs.ref()
+def hostile_answer(B, name):
+    """Return value, error number and bytes of decodes of damaged encodings of one of the CASES."""
     data = dict(CASES)[name]
     bs = max(65 * 1024, len(data))
-    enc, r, e = refs.oracle_encode_block(data, bs)
+    enc = B.encode(data, bs)[0]
     rng = np.random.default_rng(len(data))
-    for k, (venc, osz, bsz, csz) in enumerate(hostile_variants(enc, len(data), bs, rng)):
-        got_r = refs.api_decode_block(L, venc, osz, bs, buffer_size=bsz, compressed_size=csz)
-        got_o = refs.oracle_decode_block(venc, osz, bs, buffer_size=bsz, compressed_size=csz)
-        assert got_r[1:] == got_o[1:], (name, k, got_r[1:], got_o[1:])
-        if got_r[1] >= 0:
-            assert got_r[0] == got_o[0]
+    out = []
+    for venc, osz, bsz, csz in hostile_variants(enc, len(data), bs, rng):
+        dec, r, e = B.decode(venc, osz, bs, buffer_size=bsz, compressed_size=csz)
+        out.append([r, e, refs.digest(dec) if r >= 0 else None])
+    return out
 
 
-@needs_ref
+@pytest.mark.parametrize("name", HOSTILE)
+def test_hostile_decode_error_parity(name):
+    refs.check_answer(f"hostile/{name}", hostile_answer(ORACLE_BLOCKS, name))
+
+
+def medium_corpora():
+    return [synth.zipf_text(1_500_000).tobytes(), synth.source_corpus(1_500_000).tobytes(),
+            synth.mixed(1_200_000, segment=300_000).tobytes(), synth.log_stream(800_000).tobytes()]
+
+
+def medium_answer(B, datas):
+    bs = 2 << 20
+    out = []
+    for data in datas:
+        enc, r, e = B.encode(data, bs)
+        out.append([r, e, refs.digest(enc)])
+    return out
+
+
 def test_medium_corpora_block_parity():
-    L = refs.ref()
-    for gen, n in ((synth.zipf_text, 1_500_000), (synth.source_corpus, 1_500_000), (synth.mixed, 1_200_000),
-                   (synth.log_stream, 800_000)):
-        data = gen(n).tobytes() if gen is not synth.mixed else gen(n, segment=300_000).tobytes()
-        bs = 2 << 20
-        a = refs.api_encode_block(L, data, bs)
-        b = refs.oracle_encode_block(data, bs)
-        assert a == b
-        assert refs.oracle_decode_block(b[0], len(data), bs)[0] == data
+    datas = medium_corpora()
+    refs.check_answer("medium_corpora", medium_answer(ORACLE_BLOCKS, datas))
+    for data in datas:
+        assert refs.oracle_decode_block(refs.oracle_encode_block(data, 2 << 20)[0], len(data), 2 << 20)[0] == data
